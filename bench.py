@@ -17,7 +17,8 @@ pushCurrPointsToMap_, optimizeMap_.  Initialisation and keyframes are inside the
 
 A step is ONE call of mvo_vo_run_sequence (include/mvo.h: run_vo.cpp's main loop over frames in memory).
 
-One JSON line on stdout (rank 0).  Launch for N > 1:
+One JSON line on stdout (rank 0).  --dump-outputs DIR: what the last timed step returned to its caller, as .npy files (rank 0).
+Launch for N > 1:
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
       --master-port P bench.py --gpus N --steps K --warmup W
 Multi-GPU = independent sequences per GPU (replicas only, SURVEY.md §8e): NCCL only carries the per-rank timings
@@ -230,6 +231,9 @@ def run_reference(args, rank, world):
         poses, states, kf = cpu_pass(imgs)
     dt = time.perf_counter() - t0
     fps = args.steps * N_FRAMES / dt
+    if args.dump_outputs:
+        Path(args.dump_outputs).mkdir(parents=True, exist_ok=True)
+        np.save(Path(args.dump_outputs) / "poses.npy", np.asarray(poses, dtype=np.float64))
     line = {
         "impl": "reference", "metric": METRIC, "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -318,7 +322,7 @@ def run_gpu(args, rank, world, local_rank):
         vo.reset()
         a = [args_of(i) for i in range(N_FRAMES)]
         poses, infos = vo.run_sequence([x[0][0] for x in a], **a[0][1])
-        return list(poses), [inf.state_out for inf in infos], sum(inf.keyframe for inf in infos), infos[-1]
+        return list(poses), [inf.state_out for inf in infos], sum(inf.keyframe for inf in infos), infos
 
     def barrier():
         if dist is not None:
@@ -354,9 +358,12 @@ def run_gpu(args, rank, world, local_rank):
     sampler = ClockSampler(nvml_index(local_rank))
     sampler.start()
     launches0 = vo.kernel_launches
-    ms, (poses, states, kf, info_last) = timed(dev_args, args.steps)
+    ms, (poses, states, kf, infos) = timed(dev_args, args.steps)
     launches = vo.kernel_launches - launches0
     clocks = sampler.stop()
+    info_last = infos[-1]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, poses, infos, mvo_b200)
     # the dominant kernel's average launch duration: CUDA events around ITS launches only, same loop, separate pass
     kd = names.index(dominant)
     vo.timing_enable(1 << kd)
@@ -443,6 +450,18 @@ def run_gpu(args, rank, world, local_rank):
     ctx.close()
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, poses, infos, mvo_b200):
+    """The last timed step's results as a caller of mvo_vo_run_sequence receives them: poses.npy (frames x 4 x 4 camera->world)
+    and one info_<field>.npy per mvo_vo_frame_info field (frames, or frames x 16 for T_w_c_pnp), all float64 (< 100 KB)."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "poses.npy", np.asarray(poses, dtype=np.float64))
+    for name, _ in mvo_b200.VoFrameInfo._fields_:
+        if name != "pad":
+            vals = [getattr(inf, name) for inf in infos]
+            np.save(out / f"info_{name}.npy", np.array([list(v) if name == "T_w_c_pnp" else v for v in vals], dtype=np.float64))
 
 
 def bench_extras(ctx, stream, d_frames, names, torch, mvo_b200, mvo_synth):
@@ -532,7 +551,11 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (poses and per-frame results) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,7 +1,10 @@
 """Generates the committed golden vectors from the third-party code the reference calls
 (OpenCV, via the cv2 4.13 wheel in this container).  Run from the repo root:
-    python tests/golden/make_golden.py [match|orb|pnp|all]
-The reference ships no fixtures of its own (SURVEY.md §4); these pin the oracle."""
+    python tests/golden/make_golden.py [match|orb|pnp|all|run_vo_symbols|run_vo]
+The reference ships no fixtures of its own (SURVEY.md §4); these pin the oracle.  Two makers read a checkout of the reference
+that MVO_REFERENCE_DIR names and are not part of `all`: `run_vo_symbols` stores the symbols the reference's own run_vo.cpp,
+compiled against the adapter headers, needs from elsewhere; `run_vo` stores the trajectory it writes on libmvo (it needs a B200
+and oracle/_ref/run_vo_reference, which __graft_entry__.build() makes)."""
 import sys
 from pathlib import Path
 
@@ -66,6 +69,35 @@ def make_pnp():
                         cv_version=cv2.__version__)
 
 
+def make_run_vo_symbols():
+    """The undefined symbols of the reference's run_vo.cpp compiled against my_slam_adapter/include + tests/cvshim, one per line."""
+    import subprocess
+    import tempfile
+    from oracle import reference_run_vo
+    src = reference_run_vo.source()
+    assert src is not None, "MVO_REFERENCE_DIR must name a checkout of the reference"
+    with tempfile.TemporaryDirectory() as tmp:
+        obj = Path(tmp) / "run_vo.o"
+        subprocess.run(reference_run_vo.command(src, obj, compile_only=True), check=True)
+        nm = subprocess.run(["nm", "-P", "-u", str(obj)], capture_output=True, text=True, check=True).stdout
+    syms = sorted({line.split()[0] for line in nm.splitlines() if line.split()[1:2] == ["U"]})
+    (OUT / "run_vo_reference_undefined.txt").write_text("".join(s + "\n" for s in syms))
+
+
+def make_run_vo():
+    """run_vo.cpp of the reference on libmvo over the 14-frame PNG dataset of tests/test_run_vo_reference_source.py."""
+    import subprocess
+    import tempfile
+    sys.path.insert(0, str(ROOT / "tests"))
+    import test_run_vo_reference_source as t
+    from oracle import reference_run_vo
+    assert reference_run_vo.OUT.exists(), "build oracle/_ref/run_vo_reference first (MVO_REFERENCE_DIR + __graft_entry__.build())"
+    with tempfile.TemporaryDirectory() as tmp:
+        child = t.reference_child(tmp, reference_run_vo.OUT, save=t.GOLDEN_TRAJ)
+        r = subprocess.run([sys.executable, "-c", child], capture_output=True, text=True)
+        assert r.returncode == 0 and "reference run_vo child ok" in r.stdout, (r.stdout[-1500:], r.stderr[-3000:])
+
+
 if __name__ == "__main__":
     what = sys.argv[1] if len(sys.argv) > 1 else "all"
     if what in ("match", "all"):
@@ -74,3 +106,7 @@ if __name__ == "__main__":
         make_orb()
     if what in ("pnp", "all") and "make_pnp" in globals():
         make_pnp()
+    if what == "run_vo_symbols":
+        make_run_vo_symbols()
+    if what == "run_vo":
+        make_run_vo()
